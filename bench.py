@@ -153,6 +153,31 @@ def pin_to_gpu_cores(gpu_index):
     return None
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, eng, stats):
+    """Write what the last timed iteration of `value` hands its caller as float32 DIR/<name>.npy: the rollout's actions,
+    log-probabilities and values, the GAE advantages and returns, the bootstrap values, the loss statistics of every
+    minibatch update and the updated flat parameter vector.  Inputs are seeded, so two builds run with the same arguments
+    can be compared file by file.  Above DUMP_BYTES in all, the [num_steps, num_envs] arrays keep a fixed, seeded subset
+    of env columns."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    rollout = {"actions": eng.actions, "logprobs": eng.logprobs, "values": eng.values, "advantages": eng.advantages,
+               "returns": eng.returns}
+    flat = {"next_value": eng.next_value, "params": eng.flat.flat}
+    T, N = eng.T, eng.N
+    headers = 4096                                 # .npy headers, 128 bytes per file
+    room = (DUMP_BYTES - headers - 4 * sum(t.numel() for t in flat.values()) - stats["per_update"].nbytes) // (4 * len(rollout) * T)
+    cols = slice(None) if room >= N else np.sort(np.random.default_rng(0).choice(N, max(int(room), 1), replace=False))
+    for name, t in rollout.items():
+        np.save(out / f"{name}.npy", t.float().cpu().numpy()[:, cols])
+    for name, t in flat.items():
+        np.save(out / f"{name}.npy", t.float().cpu().numpy())
+    np.save(out / "update_stats.npy", stats["per_update"].astype(np.float32))
+
+
 def measured_peaks():
     p = ROOT / "MEASURED_PEAKS.json"
     if p.exists():
@@ -343,6 +368,8 @@ def run_ours(opt):
 
     replica_trace("init")
     res = timed(iteration_resident)                 # `value`: update replayed as per-epoch CUDA graphs, no profiling events
+    if opt.dump_outputs and rank == 0:
+        dump_outputs(opt.dump_outputs, eng, res["stats"])
     replica_trace("after resident loop")
     eng.update_graphs = False                       # per-kernel CUDA-event brackets cannot live inside a captured graph:
     prof_run = timed(iteration_resident, profile=True)      # the kernel table comes from an eager pass of the same iteration
@@ -698,6 +725,8 @@ def main():
     ap.add_argument("--no-extra", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-eager-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps of `value`, write what its last step computed to DIR/<name>.npy")
     opt = ap.parse_args()
     if opt.impl == "reference":
         run_reference(opt)

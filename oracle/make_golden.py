@@ -9,12 +9,15 @@ compares.  TEST INFRASTRUCTURE ONLY.
 """
 from __future__ import annotations
 
+import ast
+import hashlib
+import json
 import sys
 from pathlib import Path
 
 import numpy as np
 
-from oracle.ref_harness import run_reference
+from oracle.ref_harness import REFERENCE_ROOT, run_reference
 
 OUT = Path(__file__).resolve().parent.parent / "tests" / "golden"
 
@@ -148,6 +151,79 @@ def dqn(name, argv):
     print("wrote", name, len(losses), "updates")
 
 
+SURFACE_SCRIPTS = ["ppo.py", "ppo_atari.py", "ppo_atari_envpool.py", "ppo_atari_multigpu.py", "ppo_continuous_action.py",
+                   "dqn_atari.py", "ppo_procgen.py", "ppo_atari_lstm.py"]
+
+
+def help_digest(text):
+    """SHA-256 of a flag's help text (None when the flag has none): the fixture pins the text without holding it."""
+    return None if text is None else hashlib.sha256(text.encode()).hexdigest()
+
+
+def reference_surface(name):
+    """The public surface of each reference script: every field of its ``Args`` dataclass as [name, default, help digest]
+    (default "<expr>" where it is not a literal) and the names of its top-level classes and functions."""
+    out = {}
+    for script in SURFACE_SCRIPTS:
+        tree = ast.parse((REFERENCE_ROOT / "cleanrl" / script).read_text())
+        body = next(n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == "Args").body
+        args = []
+        for i, node in enumerate(body):
+            if isinstance(node, ast.AnnAssign):
+                try:
+                    default = ast.literal_eval(node.value)
+                except Exception:
+                    default = "<expr>"
+                doc = None
+                if i + 1 < len(body) and isinstance(body[i + 1], ast.Expr) and isinstance(body[i + 1].value, ast.Constant):
+                    doc = body[i + 1].value.value
+                args.append([node.target.id, default, help_digest(doc)])
+        out[script] = {"args": args,
+                       "module_names": [n.name for n in tree.body if isinstance(n, (ast.ClassDef, ast.FunctionDef))]}
+    (OUT / name).write_text(json.dumps(out, indent=1) + "\n")
+    print("wrote", name)
+
+
+def replay_buffer(name):
+    """cleanrl_utils/buffers.py ReplayBuffer (optimize_memory_usage=True, 50 slots) fed 137 transitions of seeded random
+    Atari frames, sampled 16 at a time (np.random.seed(t)) before and after the ring wraps.  Sampled frames are stored
+    as the index of the generated frame they equal: the stream of frames is regenerated from the same seed."""
+    from oracle import stubs
+    from cleanrl_b200.synthetic_envs import Box, Discrete
+    stubs.install()
+    sys.path.insert(0, str(REFERENCE_ROOT))
+    try:
+        from cleanrl_utils.buffers import ReplayBuffer
+        rng = np.random.default_rng(0)
+        size, at = 50, (20, 49, 50, 77, 136)
+        ref = ReplayBuffer(size, Box(0, 255, (4, 84, 84), np.uint8), Discrete(4), "cpu", optimize_memory_usage=True,
+                           handle_timeout_termination=False)
+        frames = [rng.integers(0, 256, (1, 4, 84, 84), dtype=np.uint8)]
+        rec = {k: [] for k in ("observations", "next_observations", "actions", "rewards", "dones")}
+        for t in range(137):
+            frames.append(rng.integers(0, 256, (1, 4, 84, 84), dtype=np.uint8))
+            a = rng.integers(0, 4, (1,)); r = rng.standard_normal(1).astype(np.float32); d = rng.random(1) < 0.1
+            ref.add(frames[-2], frames[-1], a, r, d, [{}])
+            if t in at:
+                st = np.random.get_state()
+                np.random.seed(t)
+                data = ref.sample(16)
+                np.random.set_state(st)
+                for k in rec:
+                    rec[k].append(getattr(data, k).numpy())
+        index = {f.tobytes(): i for i, f in enumerate(frames)}
+        out = {"sample_at": np.array(at)}
+        for k in ("observations", "next_observations"):
+            out[k + "_frame"] = np.array([[index[o.tobytes()] for o in x] for x in rec[k]])
+        for k in ("actions", "rewards", "dones"):
+            out[k] = np.stack([x.reshape(-1) for x in rec[k]])
+    finally:
+        sys.path.remove(str(REFERENCE_ROOT))
+        stubs.uninstall()
+    np.savez_compressed(OUT / name, **out)
+    print("wrote", name, {k: (v.shape, v.dtype) for k, v in out.items()})
+
+
 def main():
     OUT.mkdir(parents=True, exist_ok=True)
     only = sys.argv[1:]
@@ -169,6 +245,10 @@ def main():
         atari_envpool("ppo_procgen_n8_t16_seed2.npz",
                       ["--no-cuda", "--num-envs", "8", "--num-steps", "16", "--total-timesteps", "384", "--seed", "2",
                        "--num-minibatches", "4", "--update-epochs", "2"], 3, script="ppo_procgen.py")
+    if not only or "reference_surface" in only:
+        reference_surface("reference_cli_surface.json")
+    if not only or "replay_buffer" in only:
+        replay_buffer("replay_buffer_n50_seed0.npz")
     if "ppo_atari_full" in only:
         # ~3 CPU-minutes: generated on request only (python -m oracle.make_golden ppo_atari_full)
         atari_envpool_full("ppo_atari_envpool_n1024_t128_seed1.npz",

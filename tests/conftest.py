@@ -1,4 +1,3 @@
-import os
 import sys
 from pathlib import Path
 
@@ -13,19 +12,15 @@ GOLDEN = ROOT / "tests" / "golden"
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a real B200 (run by the driver with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
 
 
 def pytest_collection_modifyitems(config, items):
     import torch
 
     has_gpu = torch.cuda.is_available()
-    has_ref = Path(os.environ.get("CLEANRL_REFERENCE", "/root/reference")).exists()
     for item in items:
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
-        if "reference" in item.keywords and not has_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present on this box"))
 
 
 @pytest.fixture(scope="session")

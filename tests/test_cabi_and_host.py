@@ -82,7 +82,13 @@ def test_product_never_imports_oracle():
         assert not re.search(r"^\s*(from|import)\s+oracle\b", txt, flags=re.M), f"{p} imports the oracle"
 
 
-@pytest.mark.reference
+def _reference_surface(script):
+    """Args fields and top-level names of the reference script, recorded in tests/golden/reference_cli_surface.json
+    (oracle/make_golden.py reference_surface)."""
+    import json
+    return json.loads((ROOT / "tests" / "golden" / "reference_cli_surface.json").read_text())[script]
+
+
 @pytest.mark.parametrize("script,factory", [
     ("ppo.py", "ppo_args"), ("ppo_atari.py", "ppo_atari_args"), ("ppo_atari_envpool.py", "ppo_atari_envpool_args"),
     ("ppo_atari_multigpu.py", "ppo_atari_multigpu_args"), ("ppo_continuous_action.py", "ppo_continuous_action_args"),
@@ -90,50 +96,33 @@ def test_product_never_imports_oracle():
     ("ppo_atari_lstm.py", "ppo_atari_args")])
 def test_cli_fields_match_reference_args(script, factory):
     """Every reference flag exists with the same default and help text (reference Args dataclasses)."""
-    import ast
     import dataclasses
     from cleanrl_b200 import cli
-    src = Path("/root/reference/cleanrl") / script
-    tree = ast.parse(src.read_text())
-    cls = next(n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == "Args")
-    ref = {}
-    body = cls.body
-    for i, node in enumerate(body):
-        if isinstance(node, ast.AnnAssign):
-            name = node.target.id
-            try:
-                default = ast.literal_eval(node.value)
-            except Exception:
-                default = "<expr>"
-            doc = None
-            if i + 1 < len(body) and isinstance(body[i + 1], ast.Expr) and isinstance(body[i + 1].value, ast.Constant):
-                doc = body[i + 1].value.value
-            ref[name] = (default, doc)
+    from oracle.make_golden import help_digest
+    ref = {name: (default, digest) for name, default, digest in _reference_surface(script)["args"]}
+    assert ref
     ours = getattr(cli, factory)()
     fields = {f.name: f for f in dataclasses.fields(ours)}
-    for name, (default, doc) in ref.items():
+    for name, (default, digest) in ref.items():
         assert name in fields, f"{script}: flag {name} missing"
         f = fields[name]
         if default != "<expr>":
             d = f.default if f.default is not dataclasses.MISSING else f.default_factory()
             assert d == default, (name, d, default)
         helps = [m.help for m in getattr(f.type, "__metadata__", ()) if hasattr(m, "help")]
-        assert helps and helps[0] == doc, (name, helps, doc)
+        assert helps and help_digest(helps[0]) == digest, (name, helps)
     extra = set(fields) - set(ref)
     assert extra <= {"precision", "gae_kernel", "synthetic_env", "huber_loss", "env_groups"}, extra
 
 
-@pytest.mark.reference
 @pytest.mark.parametrize("script", ["ppo.py", "ppo_atari.py", "ppo_atari_envpool.py", "ppo_atari_multigpu.py",
                                     "ppo_continuous_action.py", "dqn_atari.py"])
 def test_module_level_names_match_reference(script):
     """Every top-level class / function of the reference script (what tuner.py, the eval helpers and user code
     import: Args, make_env, layer_init, Agent / QNetwork, RecordEpisodeStatistics, linear_schedule) exists in the
     drop-in module under the same name."""
-    import ast
     import importlib
-    tree = ast.parse((Path("/root/reference/cleanrl") / script).read_text())
-    names = [n.name for n in tree.body if isinstance(n, (ast.ClassDef, ast.FunctionDef))]
+    names = _reference_surface(script)["module_names"]
     mod = importlib.import_module("cleanrl_b200." + script[:-3])
     missing = [n for n in names if not hasattr(mod, n)]
     assert names and not missing, (script, missing)

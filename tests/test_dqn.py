@@ -1,6 +1,5 @@
 """DQN path (config 5): TD-loss oracle/kernels, device replay ring vs the reference's numpy ReplayBuffer,
 and the dqn_atari drop-in vs the unmodified reference run (tests/golden/dqn_atari_b8_seed1.npz)."""
-import sys
 import types
 
 import numpy as np
@@ -29,44 +28,34 @@ def test_td_loss_oracle_vs_torch():
         assert np.abs(dq - q.grad.numpy()).max() < 1e-8
 
 
-@pytest.mark.reference
 def test_replay_ring_matches_reference_replay_buffer():
     """Same adds, same numpy seed => same sampled transitions as cleanrl_utils/buffers.py ReplayBuffer
-    (optimize_memory_usage=True), before and after the ring wraps."""
-    from oracle import stubs
-    stubs.install()
-    sys.path.insert(0, "/root/reference")
-    try:
-        from cleanrl_utils.buffers import ReplayBuffer
-        from cleanrl_b200.replay import DeviceReplayRing
-        from cleanrl_b200.synthetic_envs import Box, Discrete
-        rng = np.random.default_rng(0)
-        size = 50
-        ref = ReplayBuffer(size, Box(0, 255, (4, 84, 84), np.uint8), Discrete(4), "cpu", optimize_memory_usage=True,
-                           handle_timeout_termination=False)
-        ring = DeviceReplayRing(size, (4, 84, 84), 1, torch.device("cpu"))
-        obs = rng.integers(0, 256, (1, 4, 84, 84), dtype=np.uint8)
-        for t in range(137):
-            nxt = rng.integers(0, 256, (1, 4, 84, 84), dtype=np.uint8)
-            a = rng.integers(0, 4, (1,)); r = rng.standard_normal(1).astype(np.float32); d = rng.random(1) < 0.1
-            ref.add(obs, nxt, a, r, d, [{}]); ring.add(obs, nxt, a, r, d, [{}])
-            obs = nxt
-            if t in (20, 49, 50, 77, 136):
-                st = np.random.get_state()
-                np.random.seed(t)
-                data = ref.sample(16)
-                np.random.seed(t)
-                b = ring.sample(16)
-                np.random.set_state(st)
-                assert torch.equal(ring.frames[b["rows"]], data.observations)
-                assert torch.equal(ring.frames[b["next_rows"]], data.next_observations)
-                assert torch.equal(b["actions"], data.actions.view(-1)) and torch.equal(b["rewards"], data.rewards.view(-1))
-                assert torch.equal(b["dones"], data.dones.view(-1))
-    finally:
-        sys.path.remove("/root/reference")
-        stubs.uninstall()
-        for m in [k for k in sys.modules if k.startswith("cleanrl_utils")]:
-            sys.modules.pop(m)
+    (optimize_memory_usage=True), before and after the ring wraps.  The reference's samples are recorded in
+    tests/golden/replay_buffer_n50_seed0.npz as indices into the seeded stream of frames regenerated here."""
+    from cleanrl_b200.replay import DeviceReplayRing
+    z = np.load(GOLDEN / "replay_buffer_n50_seed0.npz")
+    at = z["sample_at"].tolist()
+    assert len(at) == 5
+    rng = np.random.default_rng(0)
+    size = 50
+    ring = DeviceReplayRing(size, (4, 84, 84), 1, torch.device("cpu"))
+    frames = [rng.integers(0, 256, (1, 4, 84, 84), dtype=np.uint8)]
+    for t in range(137):
+        frames.append(rng.integers(0, 256, (1, 4, 84, 84), dtype=np.uint8))
+        a = rng.integers(0, 4, (1,)); r = rng.standard_normal(1).astype(np.float32); d = rng.random(1) < 0.1
+        ring.add(frames[-2], frames[-1], a, r, d, [{}])
+        if t in at:
+            i = at.index(t)
+            st = np.random.get_state()
+            np.random.seed(t)
+            b = ring.sample(16)
+            np.random.set_state(st)
+            want = lambda key: torch.from_numpy(np.concatenate([frames[j] for j in z[key][i]]))
+            assert torch.equal(ring.frames[b["rows"]], want("observations_frame"))
+            assert torch.equal(ring.frames[b["next_rows"]], want("next_observations_frame"))
+            assert torch.equal(b["actions"], torch.from_numpy(z["actions"][i]))
+            assert torch.equal(b["rewards"], torch.from_numpy(z["rewards"][i]))
+            assert torch.equal(b["dones"], torch.from_numpy(z["dones"][i]))
 
 
 @pytest.mark.gpu

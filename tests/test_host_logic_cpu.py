@@ -61,7 +61,8 @@ def test_host_loop_replays_reference_fixture(tmp_path, script, name):
     worker = tmp_path / "worker.py"
     worker.write_text(f"ROOT = {str(ROOT)!r}\n" + WORKER)
     out = tmp_path / "out.npz"
-    env = dict(os.environ, FIXTURE=str(GOLDEN / name), OUT=str(out), SCRIPT=script, OMP_NUM_THREADS="4")
+    # CUDA_VISIBLE_DEVICES="": the worker drives the CPU backend, so the script must take the CPU device on a GPU host too
+    env = dict(os.environ, FIXTURE=str(GOLDEN / name), OUT=str(out), SCRIPT=script, OMP_NUM_THREADS="4", CUDA_VISIBLE_DEVICES="")
     r = subprocess.run([sys.executable, str(worker)], env=env, capture_output=True, text=True, timeout=900)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-3000:]
     z, o = np.load(GOLDEN / name), np.load(out)

@@ -62,7 +62,8 @@ WORKER = textwrap.dedent('''
 def test_two_rank_gloo_data_parallel(tmp_path, module):
     script = tmp_path / "worker.py"
     script.write_text(f"ROOT = {str(ROOT)!r}\n" + WORKER)
-    env = dict(os.environ, OUT=str(tmp_path), OMP_NUM_THREADS="2", SCRIPT=module)
+    # CUDA_VISIBLE_DEVICES="": the ranks drive the CPU backend, so the script must take the CPU device on a GPU host too
+    env = dict(os.environ, OUT=str(tmp_path), OMP_NUM_THREADS="2", SCRIPT=module, CUDA_VISIBLE_DEVICES="")
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--standalone", "--nnodes=1", "--nproc-per-node=2",
                         "--local-addr", "127.0.0.1", str(script)], env=env, capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
