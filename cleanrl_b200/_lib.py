@@ -69,6 +69,7 @@ SIGNATURES = {
     "b200rl_naturecnn_bf16_workspace_bytes": (_sz, [_i64, _i]),
     "b200rl_naturecnn_bf16_pack": (_i, [_p, _i, _p, _p]),
     "b200rl_naturecnn_bf16_forward": (_i, [_p, _i, _p, _i64, _i, _p, _p, _p, _p, _p]),
+    "b200rl_naturecnn_bf16_rollout_step": (_i, [_p, _p, _p, _i64, _i, _p, _p, _p, _p, _p, _p, _p, _p]),
     "b200rl_naturecnn_bf16_backward": (_i, [_p, _p, _i, _p, _i64, _i, _p, _p, _p, _p, _p, _p, _sz, _p, _p]),
     "b200rl_frames_to_s2d_u8": (_i, [_p, _p, _i64, _p, _p, _p]),
     "b200rl_lstm_mask_state_f32": (_i, [_p, _p, _p, _i64, _i, _p, _p, _p]),

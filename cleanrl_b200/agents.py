@@ -224,6 +224,14 @@ class NatureCNNAgent(KernelAgent):
         A = self.num_actions
         return out[:, :A], out[:, A]
 
+    def rollout_step_into(self, frames, slot_rm, slot_cm, actions_out, logprobs_out, values_out, noise=None):
+        """Rollout step of the bf16 path on the uint8 rollout layout: ``frames`` (uint8 [n,4,84,84], or None when
+        ``slot_rm`` is already written) -> both slot orientations + forward + sample in one native call.  Same results
+        as ``frames_to_s2d_u8`` followed by ``sample_into`` on the slot."""
+        n, A = slot_rm.shape[0], self.num_actions
+        q = noise if noise is not None else self.noise_fn(n, A, slot_rm.device)
+        self._tc_plan().rollout_step(frames, slot_rm, slot_cm, self._flat.flat, q, actions_out, logprobs_out, values_out)
+
     def forward_train(self, b_obs, mb_inds, aux=None):
         """Minibatch forward with fused row gather (b_obs[mb_inds] never materialised); keeps activations.
         ``aux``: channel-major copy of a uint8 space-to-depth rollout (consumed by the conv1 weight gradient)."""

@@ -28,7 +28,8 @@
 //       gradient (column sums of dY) is accumulated by the four dY warps from the staged tiles.
 //   tc_gemm_tma<BN,STAGES>       fc forward / data-gradient: both operands are TMA boxes of row-major matrices.
 //   tc_wgrad_tma                 fc weight gradient (MN-major views of TMA-loaded dhid / act3 row boxes).
-//   tc_heads_*                   the A+1 head outputs in fp32 on CUDA cores.
+//   tc_heads_*                   the A+1 head outputs in fp32 on CUDA cores (tc_heads_sample: + the rollout's sampler).
+//   tc_rollout_tower<RAW>        rollout step: conv1 -> conv2 -> conv3 per image with act1 / act2 in shared memory.
 #include <cuda.h>            // CUtensorMap types only; the encoder is resolved at run time (no libcuda link)
 #include "tc_base.cuh"
 #include "tc_conv_win.cuh"
@@ -38,6 +39,7 @@
 #include "tc_reduce.cuh"
 #include "tc_aux.cuh"
 #include "tc_heads.cuh"
+#include "tc_rollout_tower.cuh"
 
 // =====================================================================================
 // Host side: NatureCNN plan over the kernels above (C-ABI entry points, include/b200rl.h)
@@ -308,6 +310,44 @@ extern "C" int b200rl_naturecnn_bf16_forward(const void* obs, int obs_format, co
       int hb = (int)ceil_div(n, 8); if (hb > num_sms() * 8) hb = num_sms() * 8;
       tc_heads_fwd<<<hb, 256, (size_t)(A + 1) * 2048, s>>>(act + Q.hid, params + L.hw, params + L.hb, n, A + 1, 512, head_out); }
     return check_launch("naturecnn/heads");
+}
+
+extern "C" int b200rl_naturecnn_bf16_rollout_step(const uint8_t* frames, uint8_t* slot_rm, uint8_t* slot_cm, int64_t n, int A,
+                                                  const float* params, const void* packed, void* acts, const float* noise,
+                                                  int64_t* action, float* logprob, float* value, void* stream) {
+    B200RL_REQUIRE(n >= 0, "naturecnn_rollout_step: negative n");
+    if (n == 0) return B200RL_OK;
+    B200RL_REQUIRE(slot_rm && params && packed && acts && noise && action && logprob && value, "naturecnn_rollout_step: null pointer");
+    B200RL_REQUIRE(!frames || slot_cm, "naturecnn_rollout_step: raw frames need the channel-major slot");
+    B200RL_REQUIRE(A >= 1 && A < kMaxHeads, "naturecnn_rollout_step: A=%d outside [1,23]", A);
+    B200RL_REQUIRE(aligned(slot_rm, 16) && aligned(acts, 16) && aligned(packed, 16) && (!frames || (aligned(frames, 16) && aligned(slot_cm, 16))),
+                   "naturecnn_rollout_step: misaligned buffer");
+    B200RL_REQUIRE(n <= (int64_t)1 << 22, "naturecnn_rollout_step: n too large");
+    const NatureLayout L(A);
+    const NatureActs Q(n, false);              // the workspace of a uint8 space-to-depth forward (format 2)
+    const bf16* P = reinterpret_cast<const bf16*>(packed);
+    bf16* act = reinterpret_cast<bf16*>(acts);
+    cudaStream_t s = (cudaStream_t)stream;
+    int rc;
+    TowerParams tp;
+    memset(&tp, 0, sizeof(tp));
+    tp.frames = frames; tp.slot_rm = slot_rm; tp.slot_cm = slot_cm; tp.n = (int)n;
+    tp.limbs = reinterpret_cast<const int8_t*>(P + L.w1l); tp.sc = reinterpret_cast<const float*>(P + L.w1sc); tp.b1 = params + L.c1b;
+    tp.w2 = P + L.w2f; tp.b2 = params + L.c2b; tp.w3 = P + L.w3f; tp.b3 = params + L.c3b; tp.act3 = act + Q.act3;
+    { ProfScope ps(s, "rollout_tower", 2.0 * n * (400 * 32 * 256 + 81 * 64 * 512 + 49 * 64 * 576),
+                   (double)n * ((frames ? 28224 * 2 + 28672 : 28224) + 3136 * 2));
+      if ((rc = launch_rollout_tower(tp, s, "naturecnn/rollout_tower"))) return rc; }
+    // fc -> hidden [n,512]: the training forward's GEMM (bit-exact with it)
+    KGemmParams p;
+    gemm_rowmajor(p, act + Q.act3, n, 49);
+    p.Bw = P + L.wfcf; p.N = 512; p.out = act + Q.hid; p.ldo = 512; p.bias = params + L.fcb; p.relu = 1;
+    { ProfScope ps(s, "fc_fwd", 2.0 * n * 512 * 3136, (double)n * (3136 + 512) * 2 + 512.0 * 3136 * 2);
+      if (n <= 8192) { if ((rc = launch_gemm_tma<64, 8>(p, s, "naturecnn/fc"))) return rc; }
+      else if ((rc = launch_gemm_tma<256, 4>(p, s, "naturecnn/fc"))) return rc; }
+    { ProfScope ps(s, "rollout_heads_sample", 2.0 * n * 512 * (A + 1), (double)n * (1024 + 4 * A + 20));
+      int hb = (int)ceil_div(n, 8); if (hb > num_sms() * 8) hb = num_sms() * 8;
+      tc_heads_sample<<<hb, 256, (size_t)(A + 1) * 2048, s>>>(act + Q.hid, params + L.hw, params + L.hb, n, A, noise, action, logprob, value); }
+    return check_launch("naturecnn/heads_sample");
 }
 
 extern "C" int b200rl_naturecnn_bf16_backward(const void* obs, const void* obs_aux, int obs_format, const int64_t* rows, int64_t n, int A,

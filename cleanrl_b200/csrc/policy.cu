@@ -8,37 +8,12 @@
 // Algorithmic bytes per sample (loss): 4*A (logits) + 4 (value) + 8 (index)
 // + 8+4*4 (action + 4 scalars) + 4*A + 4 (grads out) = 44 + 8*A.
 #include "common.cuh"
+#include "categorical.cuh"
 #include <cfloat>
 
 namespace b200rl {
 
 constexpr int kMaxA = 64;
-
-// Normalised logits / probs of one row exactly as torch builds them:
-//   lse = log(sum exp(x - max)) + max ; nl = x - lse            (Categorical ctor)
-//   p   = exp(nl - max(nl)) / sum exp(nl - max(nl))              (softmax of nl)
-struct RowStats {
-    float lse;   // logsumexp of raw logits
-    float m2;    // max of normalised logits
-    float s2;    // sum exp(nl - m2)
-};
-
-__device__ __forceinline__ RowStats row_stats(const float* __restrict__ x, int A) {
-    float m = -INFINITY;
-    for (int k = 0; k < A; ++k) m = fmaxf(m, x[k]);
-    const float mm = (fabsf(m) == INFINITY) ? 0.f : m;
-    float s = 0.f;
-    for (int k = 0; k < A; ++k) s += expf(x[k] - mm);
-    RowStats r;
-    r.lse = logf(s) + mm;
-    float m2 = -INFINITY;
-    for (int k = 0; k < A; ++k) m2 = fmaxf(m2, x[k] - r.lse);
-    float s2 = 0.f;
-    for (int k = 0; k < A; ++k) s2 += expf((x[k] - r.lse) - m2);
-    r.m2 = m2;
-    r.s2 = s2;
-    return r;
-}
 
 __global__ void __launch_bounds__(128) categorical_sample_kernel(
     const float* __restrict__ logits, int64_t ld, const float* __restrict__ noise,
@@ -50,15 +25,8 @@ __global__ void __launch_bounds__(128) categorical_sample_kernel(
     const float* x = logits + i * ld;
     const float* q = noise + i * (int64_t)A;
     const RowStats rs = row_stats(x, A);
-    float best = -INFINITY, ent = 0.f;
-    int arg = 0;
-    for (int k = 0; k < A; ++k) {
-        const float nl = x[k] - rs.lse;
-        const float p = expf(nl - rs.m2) / rs.s2;
-        const float sc = p / q[k];
-        if (sc > best) { best = sc; arg = k; }  // strict > keeps the first maximum (torch argmax)
-        ent += fmaxf(nl, -FLT_MAX) * p;
-    }
+    float ent;
+    const int arg = categorical_draw<true>(x, q, A, rs, &ent);
     action[i] = arg;
     logprob[i] = x[arg] - rs.lse;
     if (entropy) entropy[i] = -ent;

@@ -78,8 +78,8 @@ static int make_tmap_3d_u8(CUtensorMap* tm, const void* base, int64_t n_images, 
 }
 
 // uint8 frames [n_images][441 positions][64 ch] read as [n_images][221 pair rows][128 B] (image stride 28 224 B), box =
-// [1][144 rows][128 B], SWIZZLE_128B; rows >= 221 are zero-filled
-static int make_tmap_pairs_u8(CUtensorMap* tm, const void* base, int64_t n_images, const char* what) {
+// [1][box_rows][128 B], SWIZZLE_128B; rows >= 221 are zero-filled
+static int make_tmap_pairs_u8(CUtensorMap* tm, const void* base, int64_t n_images, const char* what, int box_rows = 144) {
     if (!g_encode) {
         CUtensorMap dummy;
         int rc = make_tmap_2d(&dummy, base, 128, 64, 8, what);
@@ -87,7 +87,7 @@ static int make_tmap_pairs_u8(CUtensorMap* tm, const void* base, int64_t n_image
     }
     const cuuint64_t dims[3] = {128u, 221u, (cuuint64_t)n_images};
     const cuuint64_t strides[2] = {128u, 28224u};
-    const cuuint32_t box[3] = {128u, 144u, 1u};
+    const cuuint32_t box[3] = {128u, (cuuint32_t)box_rows, 1u};
     const cuuint32_t estr[3] = {1u, 1u, 1u};
     CUresult r = g_encode(tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void*>(base), dims, strides, box, estr,
                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,

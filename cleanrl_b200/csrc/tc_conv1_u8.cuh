@@ -180,6 +180,31 @@ struct Conv1U8Params {
 // 139 pair rows per 256 output positions.  GEMM rows are pair rows; the even and the odd position of each pair get their own
 // accumulator, and a tap (dy, dx) of position p = 2q + e is the 64-byte half ((e + dx + dy) & 1) of pair row
 // q + (e + 21 dy + dx) / 2 -- a K-major SWIZZLE_128B descriptor shifted by whole rows plus a 64-byte K offset.
+// Epilogue arithmetic of conv1 on the integer tensor cores, shared by tc_conv1_i8 and the fused rollout tower
+// (tc_rollout_tower.cuh): one output position's 32 channels from its two limb accumulators.
+// y = (128 acc1 + acc2) * (s / 2^14 / 255) + bias: the limb recombination is exact in int32 (|128 acc1| < 2^31).
+// Returns the ReLU mask bits (y > 0); pk = the 32 ReLU'd bf16 outputs, packed in pairs.
+__device__ __forceinline__ uint32_t conv1_i8_epilogue(const uint32_t (&a1)[32], const uint32_t (&a2)[32], const float* s_sc,
+                                                      const float* s_bias, uint32_t (&pk)[16]) {
+    uint32_t bits = 0u;
+#pragma unroll
+    for (int c4 = 0; c4 < 32; c4 += 4) {
+        const float4 sc = *reinterpret_cast<const float4*>(s_sc + c4);
+        const float4 bi = *reinterpret_cast<const float4*>(s_bias + c4);
+        const float f0 = fmaf((float)((int)a1[c4] * 128 + (int)a2[c4]), sc.x, bi.x);
+        const float f1 = fmaf((float)((int)a1[c4 + 1] * 128 + (int)a2[c4 + 1]), sc.y, bi.y);
+        const float f2 = fmaf((float)((int)a1[c4 + 2] * 128 + (int)a2[c4 + 2]), sc.z, bi.z);
+        const float f3 = fmaf((float)((int)a1[c4 + 3] * 128 + (int)a2[c4 + 3]), sc.w, bi.w);
+        bits |= (f0 > 0.f ? 1u : 0u) << c4;
+        bits |= (f1 > 0.f ? 1u : 0u) << (c4 + 1);
+        bits |= (f2 > 0.f ? 1u : 0u) << (c4 + 2);
+        bits |= (f3 > 0.f ? 1u : 0u) << (c4 + 3);
+        pk[c4 >> 1] = pack_bf16x2_relu(f0, f1);
+        pk[(c4 >> 1) + 1] = pack_bf16x2_relu(f2, f3);
+    }
+    return bits;
+}
+
 constexpr bool kConv1I8Direct256 = true;
 template <int STAGES, int DBG>
 __global__ void __launch_bounds__(kConvWinThreads, 1) tc_conv1_i8(const __grid_constant__ CUtensorMap tmA, const Conv1U8Params p, int total_tiles) {
@@ -318,24 +343,8 @@ __global__ void __launch_bounds__(kConvWinThreads, 1) tc_conv1_i8(const __grid_c
             tc_fence_before_sync();
             __syncwarp();
             if ((tid & 31) == 0) mbar_arrive(&tempty_bar[acc]);            // accumulator drained
-            // y = (128 acc1 + acc2) * (s / 2^14 / 255) + bias: the limb recombination is exact in int32 (|128 acc1| < 2^31)
-            uint32_t bits = 0u;
             uint32_t pk[16];
-#pragma unroll
-            for (int c4 = 0; c4 < 32; c4 += 4) {
-                const float4 sc = *reinterpret_cast<const float4*>(s_sc + c4);
-                const float4 bi = *reinterpret_cast<const float4*>(s_bias + c4);
-                const float f0 = fmaf((float)((int)a1[c4] * 128 + (int)a2[c4]), sc.x, bi.x);
-                const float f1 = fmaf((float)((int)a1[c4 + 1] * 128 + (int)a2[c4 + 1]), sc.y, bi.y);
-                const float f2 = fmaf((float)((int)a1[c4 + 2] * 128 + (int)a2[c4 + 2]), sc.z, bi.z);
-                const float f3 = fmaf((float)((int)a1[c4 + 3] * 128 + (int)a2[c4 + 3]), sc.w, bi.w);
-                bits |= (f0 > 0.f ? 1u : 0u) << c4;
-                bits |= (f1 > 0.f ? 1u : 0u) << (c4 + 1);
-                bits |= (f2 > 0.f ? 1u : 0u) << (c4 + 2);
-                bits |= (f3 > 0.f ? 1u : 0u) << (c4 + 3);
-                pk[c4 >> 1] = pack_bf16x2_relu(f0, f1);
-                pk[(c4 >> 1) + 1] = pack_bf16x2_relu(f2, f3);
-            }
+            const uint32_t bits = conv1_i8_epilogue(a1, a2, s_sc, s_bias, pk);
             if (valid && !(DBG & 1)) p.mask_out[cell * 4 + cls] = bits;
             // Stores: a lane owns one output row (64 B at its own 2x2-cell address), so a direct 16-byte store instruction of
             // the warp touches 32 different lines = 32 L1 wavefronts -- measured, the epilogue's global stores took more of

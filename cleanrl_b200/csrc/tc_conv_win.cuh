@@ -50,6 +50,30 @@ __device__ __forceinline__ uint32_t pack_f16x2_sat(float lo, float hi) {
     return d;
 }
 
+// Epilogue arithmetic of the forward window convolutions, shared by tc_conv_win and the fused rollout tower
+// (tc_rollout_tower.cuh): 32 fp32 accumulators of one row -> acc * scale + bias (bias: 32 floats, global memory) ...
+__device__ __forceinline__ void win_scale_bias32(uint32_t (&v)[32], const float* bias, float scale) {
+    const float4* bp = reinterpret_cast<const float4*>(bias);
+#pragma unroll
+    for (int e = 0; e < 8; ++e) {
+        const float4 bv = __ldg(bp + e);
+        v[4 * e] = __float_as_uint(fmaf(__uint_as_float(v[4 * e]), scale, bv.x));
+        v[4 * e + 1] = __float_as_uint(fmaf(__uint_as_float(v[4 * e + 1]), scale, bv.y));
+        v[4 * e + 2] = __float_as_uint(fmaf(__uint_as_float(v[4 * e + 2]), scale, bv.z));
+        v[4 * e + 3] = __float_as_uint(fmaf(__uint_as_float(v[4 * e + 3]), scale, bv.w));
+    }
+}
+// ... -> ReLU folded into the bf16 conversion, 64 bytes of output row.
+__device__ __forceinline__ void win_pack_relu32(const uint32_t (&v)[32], int4 (&w)[4]) {
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+        w[e].x = (int)pack_bf16x2_relu(__uint_as_float(v[8 * e]), __uint_as_float(v[8 * e + 1]));
+        w[e].y = (int)pack_bf16x2_relu(__uint_as_float(v[8 * e + 2]), __uint_as_float(v[8 * e + 3]));
+        w[e].z = (int)pack_bf16x2_relu(__uint_as_float(v[8 * e + 4]), __uint_as_float(v[8 * e + 5]));
+        w[e].w = (int)pack_bf16x2_relu(__uint_as_float(v[8 * e + 6]), __uint_as_float(v[8 * e + 7]));
+    }
+}
+
 // Thread roles (576 threads): warp 0 = TMA producer; warp 1 = MMA issuer; warps 2-17 = FOUR epilogue groups of four warps
 // (one warp per TMEM lane quadrant).  Group h owns accumulator buffer h and drains tiles h, h + 4, ...
 // Why four groups: an epilogue warp runs a ~250-500 instruction dependent chain per tile (tcgen05.ld, scale/bias, ReLU
@@ -246,15 +270,7 @@ __global__ void __launch_bounds__(conv_win_threads(BN), 1) tc_conv_win(const __g
                 }
                 if (!valid || g * 32 >= p.N) continue;
                 if (p.bias) {
-                    const float4* bp = reinterpret_cast<const float4*>(p.bias + g * 32);
-#pragma unroll
-                    for (int e = 0; e < 8; ++e) {
-                        const float4 bv = __ldg(bp + e);
-                        v[4 * e] = __float_as_uint(fmaf(__uint_as_float(v[4 * e]), p.scale, bv.x));
-                        v[4 * e + 1] = __float_as_uint(fmaf(__uint_as_float(v[4 * e + 1]), p.scale, bv.y));
-                        v[4 * e + 2] = __float_as_uint(fmaf(__uint_as_float(v[4 * e + 2]), p.scale, bv.z));
-                        v[4 * e + 3] = __float_as_uint(fmaf(__uint_as_float(v[4 * e + 3]), p.scale, bv.w));
-                    }
+                    win_scale_bias32(v, p.bias + g * 32, p.scale);
                 } else {
 #pragma unroll
                     for (int e = 0; e < 32; ++e) v[e] = __float_as_uint(__uint_as_float(v[e]) * p.scale);
@@ -282,13 +298,7 @@ __global__ void __launch_bounds__(conv_win_threads(BN), 1) tc_conv_win(const __g
                         w[e].w = (int)pack_f16x2_sat(__uint_as_float(v[8 * e + 6]), __uint_as_float(v[8 * e + 7]));
                     }
                 } else if (p.relu) {
-#pragma unroll
-                    for (int e = 0; e < 4; ++e) {
-                        w[e].x = (int)pack_bf16x2_relu(__uint_as_float(v[8 * e]), __uint_as_float(v[8 * e + 1]));
-                        w[e].y = (int)pack_bf16x2_relu(__uint_as_float(v[8 * e + 2]), __uint_as_float(v[8 * e + 3]));
-                        w[e].z = (int)pack_bf16x2_relu(__uint_as_float(v[8 * e + 4]), __uint_as_float(v[8 * e + 5]));
-                        w[e].w = (int)pack_bf16x2_relu(__uint_as_float(v[8 * e + 6]), __uint_as_float(v[8 * e + 7]));
-                    }
+                    win_pack_relu32(v, w);
                 } else {
 #pragma unroll
                 for (int e = 0; e < 4; ++e) {

@@ -2,6 +2,7 @@
 #pragma once
 #include "tc_base.cuh"
 #include "tc_reduce.cuh"
+#include "categorical.cuh"
 
 namespace b200rl {
 using namespace tc;
@@ -18,6 +19,38 @@ static inline int64_t heads_rows_per_block(int64_t n) {
     return rpb;
 }
 
+// One row of the heads, computed by one warp: lane a (< A1) returns output a = hid . Wh[a] + bh[a].  Lane l holds hidden
+// units [8l, 8l+8) and [256+8l, 256+8l+8) (two 16-byte loads); sW = Wh [A1][512] in shared memory.
+__device__ __forceinline__ float heads_row(const bf16* __restrict__ hp, const float* sW, const float* __restrict__ bh, int A1, int lane) {
+    float hv[16];
+#pragma unroll
+    for (int q = 0; q < 2; ++q) {
+        const int4 v = ldg16(hp + q * 256 + lane * 8);
+        const uint32_t w[4] = {(uint32_t)v.x, (uint32_t)v.y, (uint32_t)v.z, (uint32_t)v.w};
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            hv[q * 8 + 2 * e] = __uint_as_float(w[e] << 16);
+            hv[q * 8 + 2 * e + 1] = __uint_as_float(w[e] & 0xFFFF0000u);
+        }
+    }
+    float mine = 0.f;                               // lane a keeps output a
+    for (int a = 0; a < A1; ++a) {
+        float s = 0.f;
+#pragma unroll
+        for (int q = 0; q < 2; ++q) {
+            const float4 w0 = *reinterpret_cast<const float4*>(sW + a * 512 + q * 256 + lane * 8);
+            const float4 w1 = *reinterpret_cast<const float4*>(sW + a * 512 + q * 256 + lane * 8 + 4);
+            s = fmaf(hv[q * 8 + 0], w0.x, s); s = fmaf(hv[q * 8 + 1], w0.y, s);
+            s = fmaf(hv[q * 8 + 2], w0.z, s); s = fmaf(hv[q * 8 + 3], w0.w, s);
+            s = fmaf(hv[q * 8 + 4], w1.x, s); s = fmaf(hv[q * 8 + 5], w1.y, s);
+            s = fmaf(hv[q * 8 + 6], w1.z, s); s = fmaf(hv[q * 8 + 7], w1.w, s);
+        }
+        s = warp_sum(s);
+        if (lane == a) mine = s + bh[a];
+    }
+    return mine;
+}
+
 // out[n][A1] = hidden[n][512](bf16) . Wh[A1][512]^T + bh.  One warp per row: lane l holds hidden units
 // [8l, 8l+8) and [256+8l, 256+8l+8) (two 16-byte loads), weights are read as float4 from shared memory.
 __global__ void __launch_bounds__(256) tc_heads_fwd(const bf16* __restrict__ hid, const float* __restrict__ Wh,
@@ -28,34 +61,37 @@ __global__ void __launch_bounds__(256) tc_heads_fwd(const bf16* __restrict__ hid
     __syncthreads();
     const int lane = threadIdx.x & 31, wpb = blockDim.x >> 5;
     for (int64_t row = (int64_t)blockIdx.x * wpb + (threadIdx.x >> 5); row < n; row += (int64_t)gridDim.x * wpb) {
-        float hv[16];
-        const bf16* hp = hid + row * 512;
-#pragma unroll
-        for (int q = 0; q < 2; ++q) {
-            const int4 v = ldg16(hp + q * 256 + lane * 8);
-            const uint32_t w[4] = {(uint32_t)v.x, (uint32_t)v.y, (uint32_t)v.z, (uint32_t)v.w};
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                hv[q * 8 + 2 * e] = __uint_as_float(w[e] << 16);
-                hv[q * 8 + 2 * e + 1] = __uint_as_float(w[e] & 0xFFFF0000u);
-            }
-        }
-        float mine = 0.f;                               // lane a keeps output a
-        for (int a = 0; a < A1; ++a) {
-            float s = 0.f;
-#pragma unroll
-            for (int q = 0; q < 2; ++q) {
-                const float4 w0 = *reinterpret_cast<const float4*>(sW + a * 512 + q * 256 + lane * 8);
-                const float4 w1 = *reinterpret_cast<const float4*>(sW + a * 512 + q * 256 + lane * 8 + 4);
-                s = fmaf(hv[q * 8 + 0], w0.x, s); s = fmaf(hv[q * 8 + 1], w0.y, s);
-                s = fmaf(hv[q * 8 + 2], w0.z, s); s = fmaf(hv[q * 8 + 3], w0.w, s);
-                s = fmaf(hv[q * 8 + 4], w1.x, s); s = fmaf(hv[q * 8 + 5], w1.y, s);
-                s = fmaf(hv[q * 8 + 6], w1.z, s); s = fmaf(hv[q * 8 + 7], w1.w, s);
-            }
-            s = warp_sum(s);
-            if (lane == a) mine = s + bh[a];
-        }
+        const float mine = heads_row(hid + row * 512, sW, bh, A1, lane);
         if (lane < A1) out[row * A1 + lane] = mine;     // one coalesced store per row
+    }
+}
+// Rollout step: heads + Categorical sample in one pass, one warp per row.  The A + 1 outputs are tc_heads_fwd's
+// (heads_row), the draw is categorical_sample_kernel's (row_stats + categorical_draw on the same fp32 logits), so action,
+// log-probability and value equal the two-kernel chain bit for bit; no [n, A+1] round trip through global memory and no
+// entropy (the rollout does not store it).  noise: Exp(1) draws [n, A].
+__global__ void __launch_bounds__(256) tc_heads_sample(const bf16* __restrict__ hid, const float* __restrict__ Wh,
+                                                       const float* __restrict__ bh, int64_t n, int A,
+                                                       const float* __restrict__ noise, int64_t* __restrict__ action,
+                                                       float* __restrict__ logprob, float* __restrict__ value) {
+    extern __shared__ float sW[];                       // [A1][512]
+    __shared__ float sX[8][kMaxHeads];                  // one row of outputs per warp
+    const int A1 = A + 1;
+    for (int i = threadIdx.x; i < A1 * 512; i += blockDim.x) sW[i] = Wh[i];
+    __syncthreads();
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, wpb = blockDim.x >> 5;
+    float* x = sX[wid];
+    for (int64_t row = (int64_t)blockIdx.x * wpb + wid; row < n; row += (int64_t)gridDim.x * wpb) {
+        const float mine = heads_row(hid + row * 512, sW, bh, A1, lane);
+        if (lane < A1) x[lane] = mine;
+        __syncwarp();
+        if (lane == 0) {
+            const RowStats rs = row_stats(x, A);
+            const int arg = categorical_draw<false>(x, noise + row * (int64_t)A, A, rs, nullptr);
+            action[row] = arg;
+            logprob[row] = x[arg] - rs.lse;
+            value[row] = x[A];
+        }
+        __syncwarp();
     }
 }
 // dhid_pre[n][512] (bf16) = (dhead[n][A1] . Wh[A1][512]) * (hid > 0).  Thread = 8 consecutive hidden units of one

@@ -509,6 +509,33 @@ class NatureCNNBf16:
         _lib.check(rc, "naturecnn_bf16_forward")
         return head_out
 
+    def rollout_step(self, frames, slot_rm, slot_cm, flat_params, noise, action, logprob, value):
+        """One rollout policy step on the uint8 rollout layout in one native call (conv tower -> fc -> heads + sampler):
+        ``frames`` uint8 [n,4,84,84] are converted into both slot orientations (``slot_rm`` [n,441,64], ``slot_cm``
+        [n,64,448]) on the way; ``frames=None``: ``slot_rm`` already holds them.  Writes ``action`` (int64),
+        ``logprob`` and ``value`` [n]; bit-identical to frames_to_s2d_u8 + forward + categorical_sample."""
+        lib = _lib.load()
+        n = slot_rm.shape[0]
+        _contig(slot_rm, "slot_rm")
+        if tuple(slot_rm.shape[1:]) != (441, 64) or slot_rm.dtype != torch.uint8:
+            raise TypeError(f"slot_rm must be uint8 [n,441,64] (got {slot_rm.dtype} {tuple(slot_rm.shape)})")
+        if frames is not None:
+            _contig(frames, "frames"); _contig(slot_cm, "slot_cm")
+            if tuple(frames.shape) != (n, 4, 84, 84) or tuple(slot_cm.shape) != (n, 64, 448):
+                raise ValueError("frames [n,4,84,84] and slot_cm [n,64,448] must match slot_rm's n")
+        _contig(noise, "noise")
+        assert tuple(noise.shape) == (n, self.A)
+        for nm, t in (("action", action), ("logprob", logprob), ("value", value)):
+            _contig(t, nm)
+            assert t.shape[0] == n, nm
+        f = torch.float32
+        rc = lib.b200rl_naturecnn_bf16_rollout_step(
+            _ptr(frames, torch.uint8, "frames", True), _ptr(slot_rm, torch.uint8, "slot_rm"),
+            _ptr(slot_cm if frames is not None else None, torch.uint8, "slot_cm", True), n, self.A,
+            _ptr(flat_params, f, "params"), self.packed.data_ptr(), self.acts(n, 2).data_ptr(), _ptr(noise, f, "noise"),
+            _ptr(action, torch.int64, "action"), _ptr(logprob, f, "logprob"), _ptr(value, f, "value"), _stream())
+        _lib.check(rc, "naturecnn_bf16_rollout_step")
+
     def grad_tail_offset(self):
         """Element offset from which the flat gradient (fc + heads, 95 % of it) is final when ``tail_event`` fires."""
         return int(_lib.load().b200rl_naturecnn_grad_tail_offset(self.A))

@@ -209,17 +209,31 @@ class PPOEngine:
             dst.copy_(src, non_blocking=True)
         self.h2d_bytes += src.numel() * src.element_size()
 
+    def _fused_rollout(self):
+        """uint8 rollout layout with an agent that has the one-call rollout step (conv tower + fc + heads/sampler)."""
+        return self.u8_rollout and getattr(self.agent, "precision", "fp32") == "bf16" and hasattr(self.agent, "rollout_step_into")
+
+    def _rollout_step(self, step, src_u8, sl=slice(None), noise=None):
+        """Policy step of rows ``sl`` of slot ``step``: ``src_u8`` = their uint8 NCHW frames (None: the slot already holds
+        them).  One native call on the u8 rollout layout; otherwise storage conversion, then forward + sampler."""
+        if self._fused_rollout():
+            self.agent.rollout_step_into(src_u8, self.obs[step][sl], self.obs_t[step][sl], self.actions[step][sl],
+                                         self.logprobs[step][sl], self.values[step][sl], noise=noise)
+            return
+        if src_u8 is not None:
+            self._to_storage(src_u8, step, sl)
+        self.agent.sample_into(self.obs[step][sl], self.actions[step][sl], self.logprobs[step][sl], self.values[step][sl],
+                               noise=noise)
+
     def _step_device_work(self, step, noise=None):
         """Everything a policy step does on the device after the observation batch has landed."""
         if self.s2d:
-            self._to_storage(self.obs_u8, step)
+            return self._rollout_step(step, self.obs_u8, noise=noise)
         self.agent.sample_into(self.obs[step], self.actions[step], self.logprobs[step], self.values[step], noise=noise)
 
     def _chunk_device_work(self, step, c):
         sl = slice(*self.chunk_bounds[c])
-        self._to_storage(self.obs_u8[sl], step, sl)
-        self.agent.sample_into(self.obs[step][sl], self.actions[step][sl], self.logprobs[step][sl],
-                               self.values[step][sl], noise=self.noise_buf[sl])
+        self._rollout_step(step, self.obs_u8[sl], sl, noise=self.noise_buf[sl])
 
     def _run_step(self, step, chunk=None):
         if chunk is not None:
@@ -320,9 +334,9 @@ class PPOEngine:
             for step in range(self.T):
                 src = obs_pool[step % P]
                 if self.s2d and src.dtype == torch.uint8:
-                    self._to_storage(src, step)
-                else:
-                    self.obs[step].copy_(src)
+                    self._rollout_step(step, src)
+                    continue
+                self.obs[step].copy_(src)
                 self.agent.sample_into(self.obs[step], self.actions[step], self.logprobs[step], self.values[step])
 
         if not getattr(self.agent, "graph_friendly", False):
@@ -378,7 +392,7 @@ class PPOEngine:
     def _part_work(self, step, lo, hi):
         sl = slice(lo, hi)
         if self.s2d:
-            self._to_storage(self.obs_u8[sl], step, sl)
+            return self._rollout_step(step, self.obs_u8[sl], sl, noise=self._noise_bufs[step & 1][sl])
         self.agent.sample_into(self.obs[step][sl], self.actions[step][sl], self.logprobs[step][sl], self.values[step][sl],
                                noise=self._noise_bufs[step & 1][sl])
 
@@ -453,8 +467,7 @@ class PPOEngine:
             ops.frames_delta_s2d_u8(self._new_d[sl], prev_rm[sl], prev_cm[sl], dst_rm[sl], dst_cm[sl],
                                     full_slot=self._slot_d[sl], full_frames=self._delta[part]["full_d"])
         if sample:
-            self.agent.sample_into(dst_rm[sl], self.actions[step][sl], self.logprobs[step][sl], self.values[step][sl],
-                                   noise=self._noise_bufs[step & 1][sl])
+            self._rollout_step(step, None, sl, noise=self._noise_bufs[step & 1][sl])
 
     @staticmethod
     def _host_pinned(arr):

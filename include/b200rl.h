@@ -341,6 +341,15 @@ int b200rl_naturecnn_bf16_pack(const float* params, int A, void* packed, void* s
 int b200rl_naturecnn_bf16_forward(const void* obs, int obs_format, const int64_t* rows, int64_t n, int A,
                                   const float* params, const void* packed, void* acts,
                                   float* head_out, void* stream);
+/* One rollout policy step of the bf16 NatureCNN on the uint8 rollout layout: conv tower (conv1..conv3 per image in
+ * shared memory) -> fc -> heads + Categorical sample, writing action / logprob / value of n rows.  frames != NULL: uint8
+ * [n,4,84,84] frames, both slot orientations (slot_rm [n,441,64], slot_cm [n,64,448]) are written from them; frames ==
+ * NULL: slot_rm already holds the space-to-depth frames (slot_cm unused).  acts: the workspace of
+ * b200rl_naturecnn_bf16_acts_bytes(n, B200RL_OBS_S2D_U8); noise: Exp(1) draws [n, A].  Same results, bit for bit, as
+ * b200rl_frames_to_s2d_u8 + b200rl_naturecnn_bf16_forward + b200rl_categorical_sample_f32. */
+int b200rl_naturecnn_bf16_rollout_step(const uint8_t* frames, uint8_t* slot_rm, uint8_t* slot_cm, int64_t n, int A,
+                                       const float* params, const void* packed, void* acts, const float* noise,
+                                       int64_t* action, float* logprob, float* value, void* stream);
 int b200rl_naturecnn_bf16_backward(const void* obs, const void* obs_aux, int obs_format, const int64_t* rows, int64_t n, int A,
                                    const float* params, const void* packed, void* acts,
                                    const float* dhead, float* grads,
